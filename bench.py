@@ -26,11 +26,17 @@ roofline = tsc_step_kernel: algorithmic bytes (BASELINE.md §3 formula with the 
 cpu_baseline / --impl reference = the CPU port of the SAME work (SUMO + TF1 are absent): oracle/tsc_sim_ref.c on all
         usable host threads (cgroup cpu.max respected) for the control step and, in train mode, oracle/learner_cpu.py
         (torch CPU fp32, all threads) for the policy forward of every step and one n-step A2C update per n_step —
-        a bounded sample of replicas, named in `sample`.
+        a bounded sample of replicas, named in `sample`.  --impl reference times exactly --steps control steps after
+        the burn-in, which must both fit in one episode (past its end the network drains: a different workload); the
+        cpu_baseline of our arm times the same --steps, cut at the episode end, and reports its count in `steps`.
 --scenario real_net = BASELINE configs[3] (Monaco, 28 agents, MA2C, 2048 replicas, n_step 40,
         config/config_ma2c_real.ini); the default large_grid = configs[2].
 value_steady = the same metric with the update amortised over n_step control steps (the driver's short --steps
         window is forced to contain one whole update, which over-weights it; both numbers are printed).
+--dump-outputs DIR = after the timed steps, what the timed path computed in its last step is written as DIR/<name>.npy
+        (float32, see last_step_outputs); inputs are seeded, so two builds run with the same arguments can be compared
+        output for output.  Our arm only: --impl reference times the CPU oracle on its own replica sample and
+        inputs, with the learner's share timed apart from the simulator, so it has no last step to compare.
 """
 import argparse
 import json
@@ -89,7 +95,14 @@ def parse():
     p.add_argument("--policy", default="lstm", choices=["lstm", "fc"], help="fc = FcACPolicy (agents/policies.py:214-256)")
     p.add_argument("--e2e-parts", type=int, default=4,
                    help="replica ranges of the host-buffer (e2e) loop, one stream each (1: single blocking tsc_step_host)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write what the timed path computed in its last timed step as DIR/<name>.npy")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        p.error("--dump-outputs writes the outputs of the device path (--impl ours)")
+    return p, args
 
 
 def workload_name(R, mode, agent="ma2c", policy="lstm", scenario="large_grid"):
@@ -167,9 +180,56 @@ def make_layout(net, args):
                         ff=64 if args.agent == "ma2c" else 0, h=64, max_na=net.max_na, recurrent=args.policy != "fc")
 
 
-def cpu_reference(net, par, args, threads, n_step, mode, budget_s=12.0):
+DUMP_REPLICAS = 1024          # per-replica outputs are dumped for a fixed sample of this many replicas
+DUMP_MAX_BYTES = 64 << 20
+
+
+def last_step_outputs(sim, trainer):
+    """What the timed path handed its caller in its last step, as host float32 arrays.
+    train: the weights after the step's A2C update (the timed region always ends on one), the per-agent gradient norms
+           of that update, and the step's transition: next observation, normalised / clipped reward, sampled actions,
+           value estimates.
+    sim:   what tsc_step returned: observation, per-agent reward, global reward, done.
+    Per-replica arrays keep the replicas of a fixed, seeded sample (at most DUMP_REPLICAS, in ascending order), listed
+    in `replicas`."""
+    import torch
+    rows = np.sort(np.random.default_rng(0).choice(sim.R, min(sim.R, DUMP_REPLICAS), replace=False))
+    idx = torch.from_numpy(rows).to(sim.device)
+    host = lambda x: x.index_select(0, idx).float().cpu().numpy()
+    if trainer is not None:
+        m = trainer.model
+        assert m.t == 0, "the timed region must end on an update"
+        out = {"params": m.P.cpu().numpy(), "grad_norms": m.norms.cpu().numpy(), "obs": host(m.obs_hist[m.T]),
+               "reward": host(m.rew_hist[m.T - 1]), "action": host(m.act_hist[m.T - 1]),
+               "value": host(m.val_hist[m.T - 1])}
+    else:
+        out = {"obs": host(sim.obs), "reward": host(sim.reward), "global_reward": host(sim.greward),
+               "done": host(sim.done)}
+    out["replicas"] = rows.astype(np.float32)
+    assert sum(a.nbytes for a in out.values()) <= DUMP_MAX_BYTES
+    return out
+
+
+def episode_steps(par):
+    return par.episode_length_sec // par.control_interval_sec
+
+
+def sim_mode_inputs(net, R, dev, rank, n_act_sets=16):
+    """Seeded device inputs of --mode sim: `n_act_sets` sets of uniform-random actions (step i of each phase plays set
+    i % n_act_sets) and one set of fingerprints."""
+    import torch
+    gen = torch.Generator(device=dev)
+    gen.manual_seed(1234 + rank)
+    n_a_dev = torch.tensor(net.n_a_ls, device=dev, dtype=torch.int64)
+    acts = [(torch.randint(0, 1 << 30, (R, net.n_nodes), device=dev, generator=gen) % n_a_dev).to(torch.int32)
+            for _ in range(n_act_sets)]
+    fp = torch.rand(R, net.n_nodes, net.max_na, device=dev, generator=gen)
+    return acts, fp
+
+
+def cpu_reference(net, par, args, threads, n_step, mode, n_t, budget_s=12.0):
     """Time the CPU port on `threads` host threads over a bounded sample of the workload: R_cpu replicas, burn-in to the
-    same simulated time, then timed control steps of the simulator (oracle/tsc_sim_ref.c, pthreads over replicas); in
+    same simulated time, then n_t timed control steps of the simulator (oracle/tsc_sim_ref.c, pthreads over replicas); in
     train mode the learner's share of the same steps is timed too (oracle/learner_cpu.py: policy forward of every step,
     one n-step update per n_step steps) and added — the reference runs env and learner serially (utils.py:142-193)."""
     from oracle.sim_ref import RefSim
@@ -185,7 +245,6 @@ def cpu_reference(net, par, args, threads, n_step, mode, budget_s=12.0):
     for _ in range(40):
         pilot.step(acts_of(threads), None, threads=threads)
     c_step = (time.perf_counter() - t0) / 40            # seconds per (threads replicas) step
-    n_t = int(min(max(args.steps, 60), 240))             # timed control steps (stay inside the episode)
     R_cpu = int(np.clip(budget_s / ((args.burnin + n_t) * c_step * 3.0) * threads, threads, 4096))
     R_cpu = max(threads, R_cpu // threads * threads)
     sim = RefSim(net, par, R_cpu)
@@ -212,7 +271,7 @@ def cpu_reference(net, par, args, threads, n_step, mode, budget_s=12.0):
                         "(measured on %d replicas: %.2f s, scaled x%.1f) on torch CPU fp32, %d threads"
                         % (R_cpu, n_t, el_fwd, n_t, n_step, R_upd, t_upd, R_cpu / R_upd, threads))
     return {"value": R_cpu * net.n_nodes * n / el, "unit": "agent-env-steps/s", "cores": threads,
-            "kind": "port",
+            "kind": "port", "steps": n,
             "sample": "%d replicas x %d control steps after %d burn-in steps (mean live %.0f veh/replica): "
                       "oracle/tsc_sim_ref.c on %d pthreads (%.2f s) %s; SUMO + TF1 are absent from the image, so this is "
                       "the CPU port of the same work, not SUMO / TensorFlow"
@@ -221,7 +280,7 @@ def cpu_reference(net, par, args, threads, n_step, mode, budget_s=12.0):
 
 
 def main():
-    args = parse()
+    parser, args = parse()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -236,10 +295,12 @@ def main():
 
     # ---------------- reference arm: the CPU implementation of the path ----------------------
     if args.impl == "reference":
+        if args.burnin + args.steps > episode_steps(par):
+            parser.error("--burnin + --steps = %d control steps: the episode has %d"
+                         % (args.burnin + args.steps, episode_steps(par)))
         if rank != 0:
             return
-        t_steps = max(args.steps, 1)
-        cb, n, el, R_cpu = cpu_reference(net, par, args, cores, n_step, mode, budget_s=args.cpu_budget)
+        cb, n, el, R_cpu = cpu_reference(net, par, args, cores, n_step, mode, args.steps, budget_s=args.cpu_budget)
         line = {"impl": "reference", "metric": "agent-env-steps/sec", "value": cb["value"],
                 "unit": "agent-env-steps/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
                 "ms_per_step": 1e3 * el / n, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -298,19 +359,13 @@ def main():
         from deeprl_signal_control_b200.dist import shard_replicas
         _, _, seeds = shard_replicas(rank, world, R, args.seed)
         sim.reset(seeds)
-        gen = torch.Generator(device=dev)
-        gen.manual_seed(1234 + rank)
-        n_act_sets = 16
-        n_a_dev = torch.tensor(net.n_a_ls, device=dev, dtype=torch.int64)
-        acts = [(torch.randint(0, 1 << 30, (R, net.n_nodes), device=dev, generator=gen) % n_a_dev).to(torch.int32)
-                for _ in range(n_act_sets)]
-        fp = torch.rand(R, net.n_nodes, net.max_na, device=dev, generator=gen)
+        acts, fp = sim_mode_inputs(net, R, dev, rank)
         sim_events = []
 
         def one_step(i):
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            sim.step(acts[i % n_act_sets], fp)
+            sim.step(acts[i % len(acts)], fp)
             e1.record()
             sim_events.append((e0, e1))
 
@@ -342,6 +397,8 @@ def main():
         one_step(i)
     t_end.record()
     barrier()
+    # before the e2e loop below steps the same simulator / learner further
+    dumped = last_step_outputs(sim, trainer) if args.dump_outputs and rank == 0 else None
     total_ms = t_start.elapsed_time(t_end)
     evs = trainer.sim_events if trainer is not None else sim_events
     kern_ms = float(np.mean([a.elapsed_time(b) for a, b in evs]))
@@ -490,7 +547,8 @@ def main():
                         "state per vehicle) - see `issue` and DESIGN.md section 5"}
     cb = None
     if not args.no_cpu_baseline:
-        cb, _, _, _ = cpu_reference(net, par, args, cores, n_step, mode, budget_s=args.cpu_budget)
+        n_cpu = max(1, min(args.steps, episode_steps(par) - args.burnin))
+        cb, _, _, _ = cpu_reference(net, par, args, cores, n_step, mode, n_cpu, budget_s=args.cpu_budget)
     line = {"metric": "agent-env-steps/sec", "value": value, "unit": "agent-env-steps/s", "n_gpus": world,
             "steps": args.steps, "warmup": max(args.warmup, 3), "ms_per_step": total_ms_max / args.steps,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -514,6 +572,10 @@ def main():
                     "windows_ms": e2e_windows_all},
             "gpu_launches": timed_launches,
             "roofline": roofline, "cpu_baseline": cb}
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -42,3 +42,22 @@ def test_reference_arm_covers_the_learner_and_the_monaco_scenario():
     assert "policy forward" in s and "A2C update" in s and "tsc_sim_ref.c" in s
     assert d["cpu_baseline"]["sim_only_value"] > d["value"] > 0
     assert d["cpu_baseline"]["cores"] <= len(os.sched_getaffinity(0))
+
+
+def test_reference_arm_times_the_steps_it_reports():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "7",
+                          "--warmup", "3", "--burnin", "20", "--cpu-budget", "1.0", "--mode", "sim"],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads([l for l in out.stdout.splitlines() if l.strip()][0])
+    cb = d["cpu_baseline"]
+    assert d["steps"] == cb["steps"] == 7 and " x 7 control steps after 20 burn-in steps" in cb["sample"]
+
+
+def test_arguments_that_would_time_or_dump_nothing_are_rejected(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)],
+                  ["--impl", "reference", "--burnin", "240", "--steps", "481"]):     # 721 steps: past the 720-step episode
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                             timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and "error" in out.stderr and not out.stdout.strip(), extra
+    assert not os.listdir(tmp_path)

@@ -1,7 +1,8 @@
 """CPU: general SUMO ingest (net/sumo_ingest.py, SURVEY 8f.2): signal programs, neighbour map and demand are read from
 scenario FILES.  (1) a synthetic two-junction scenario written by tests/fixtures/make_mini_sumo.py loads, routes, and
-runs in the oracle with vehicle conservation; (2) when the reference checkout is present, the Monaco scenario ingested
-from most.net.xml + a route file written by the reference's own generator equals the hand-wired Monaco tables."""
+runs in the oracle with vehicle conservation; (2) the Monaco scenario ingested from the reference's most.net.xml + a
+route file written by the reference's own generator equals the hand-wired Monaco tables."""
+import lzma
 import os
 import sys
 
@@ -63,22 +64,19 @@ def test_mini_scenario_runs_in_the_oracle(tmp_path):
     assert m["arrived"] > 250 and bool(d[0])
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/real_net/data/in/most.net.xml"), reason="needs the reference checkout")
 def test_monaco_from_files_equals_the_hand_wired_scenario(tmp_path):
     """most.net.xml + the route file the reference's generator writes (real_net/data/build_file.py:output_flows) +
     the reference's phase sets and neighbour lists -> the same tables as net/real_net.py's Monaco definition; the
-    tlLogic programs of the net file themselves yield an action set for each of the 28 agents as well."""
-    import types
+    tlLogic programs of the net file themselves yield an action set for each of the 28 agents as well.
+    Both files are stored under tests/golden: monaco_most.net.xml.xz is the reference's real_net/data/in/most.net.xml
+    (xz-compressed, byte-identical once unpacked) and monaco_most_325.rou.xml is output_flows(325, seed=None)."""
     from deeprl_signal_control_b200.net import real_net as rn, sumo_ingest as ing
-    sys.path.insert(0, "/root/reference")
-    for name in ("traci", "sumolib"):
-        sys.modules.setdefault(name, types.ModuleType(name))
-    import importlib
-    bf = importlib.import_module("real_net.data.build_file")
-    rou = tmp_path / "most.rou.xml"
-    rou.write_text(bf.output_flows(325, seed=None))
-    net_file = "/root/reference/real_net/data/in/most.net.xml"
-    a = ing.load_sumo_scenario(net_file, str(rou), tls_phases={n: rn.PHASES[v[0]] for n, v in rn.NODES.items()},
+    gold = os.path.join(ROOT, "tests", "golden")
+    rou = os.path.join(gold, "monaco_most_325.rou.xml")
+    net_file = str(tmp_path / "most.net.xml")
+    with lzma.open(os.path.join(gold, "monaco_most.net.xml.xz"), "rb") as src, open(net_file, "wb") as dst:
+        dst.write(src.read())
+    a = ing.load_sumo_scenario(net_file, rou, tls_phases={n: rn.PHASES[v[0]] for n, v in rn.NODES.items()},
                                neighbor_map={k: list(v[1]) for k, v in rn.NODES.items()}, agent="ma2c")
     b = rn.real_net_tables("ma2c")
     # routes (hence lane / link numbering) come in file order there and in FLOWS order here: compare by NAME
