@@ -21,7 +21,9 @@ SYMBOLS = ["tsc_last_error", "tsc_create", "tsc_destroy", "tsc_reset", "tsc_set_
            # include/tsc_learn.h
            "tscl_create", "tscl_destroy", "tscl_fc_embed", "tscl_lstm_seq_fwd", "tscl_heads", "tscl_returns",
            "tscl_heads_loss", "tscl_lstm_seq_bwd", "tscl_fc_bwd", "tscl_fc_bwd_tc", "tscl_wgrad_tc", "tscl_clip_rmsprop",
-           "tscl_pack_weights", "tscl_policy_step", "tscl_policy_step_v2", "tscl_policy_step_v2r", "tscl_unpack_store", "tscl_pack_wht", "tscl_lstm_seq_bwd_tc", "tscl_pack_wxt", "tscl_lstm_seq_bwd_tc_dx", "tscl_dx_tc", "tscl_host_transition", "tscl_device_transition", "tscl_memcpy_async", "tscl_fc_hidden_fwd", "tscl_fc_hidden_bwd", "tscl_debug_policy_prof", "tscl_debug_bptt_prof"]
+           "tscl_pack_weights", "tscl_policy_step", "tscl_policy_step_v2", "tscl_policy_step_v2r", "tscl_unpack_store", "tscl_pack_wht", "tscl_lstm_seq_bwd_tc", "tscl_pack_wxt", "tscl_lstm_seq_bwd_tc_dx", "tscl_dx_tc", "tscl_host_transition", "tscl_device_transition", "tscl_memcpy_async", "tscl_fc_hidden_fwd", "tscl_fc_hidden_bwd", "tscl_debug_policy_prof", "tscl_debug_bptt_prof",
+           "tscl_iql_create", "tscl_iql_destroy", "tscl_iql_forward", "tscl_iql_sample", "tscl_iql_td_grad",
+           "tscl_iql_clip_adam", "tscl_iql_transition"]
 
 
 def build_native(force: bool = False, verbose: bool = False) -> str:

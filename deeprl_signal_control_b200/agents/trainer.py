@@ -226,3 +226,74 @@ class BatchedTrainer:
     def run(self, n_control_steps: int):
         for _ in range(n_control_steps):
             self.control_step()
+
+
+class BatchedIQLTrainer:
+    """The episode protocol of `BatchedTrainer` for `BatchedIQL` (reference utils.py:Trainer.explore/run with an IQL
+    model): per control step epsilon-greedy forward -> env.step -> add_transition; backward() every batch_size steps and
+    at an episode end; per episode env.reset() with fresh seeds.  The simulator reads its actions from the ring's action
+    slot and writes the next observation straight into the ring's observation slot.
+
+    At an episode end the reset observation overwrites the terminal next observation of the last transition (both
+    live in the same ring slot).  That is harmless: the transition is stored with done = True, whose TD target is r."""
+
+    def __init__(self, sim: BatchedSim, model, seed0: int = 12):
+        import torch.distributed as tdist
+        assert not (tdist.is_available() and tdist.is_initialized() and tdist.get_world_size() > 1), \
+            "BatchedIQLTrainer runs on one rank (no gradient all-reduce yet)"
+        assert model.R == sim.R and model.C > 0
+        self.sim, self.model = sim, model
+        self.seed0 = int(seed0)
+        self.episode = 0
+        self.T_episode = int(np.ceil(sim.params.episode_length_sec / sim.params.control_interval_sec))
+        self.step_in_episode = 0
+        self.episode_rewards = []
+        self._rew_acc = torch.zeros(sim.R, device=sim.device)
+        self.n_env_steps = 0
+        self.n_updates = 0
+        self.fwd_events = None        # lists of (start, end) CUDA events around forward / tsc_step / backward
+        self.sim_events = None
+        self.update_events = None
+        self.start_episode()
+
+    def start_episode(self):
+        sim, m = self.sim, self.model
+        seeds = _dist.episode_seeds(self.seed0, self.episode, m.replica0, sim.R, sim.R)
+        self.episode += 1
+        sim.reset(seeds)
+        sim.set_train_mode(True)
+        m.reset()
+        sim.observe(None, obs_out=m.obs_slot())
+        self.step_in_episode = 0
+        self._rew_acc.zero_()
+
+    @staticmethod
+    def _timed(events, fn):
+        if events is None:
+            return fn()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        out = fn()
+        e1.record()
+        events.append((e0, e1))
+        return out
+
+    def control_step(self):
+        sim, m = self.sim, self.model
+        act = self._timed(self.fwd_events, lambda: m.forward())
+        _, reward, greward, _ = self._timed(self.sim_events,
+                                            lambda: sim.step(act, None, obs_out=m.obs_slot(m.n_total + 1)))
+        self.step_in_episode += 1
+        done = self.step_in_episode >= self.T_episode                # lock-step: envs/env.py:577-579
+        m.add_transition(reward, greward, self._rew_acc, done)
+        self.n_env_steps += 1
+        if done or self.step_in_episode % m.n_step == 0:             # utils.py:Trainer.explore returns -> backward
+            if self._timed(self.update_events, lambda: m.backward()):
+                self.n_updates += 1
+        if done:
+            self.episode_rewards.append(float((self._rew_acc / self.T_episode).mean()))   # utils.py:296-305
+            self.start_episode()
+
+    def run(self, n_control_steps: int):
+        for _ in range(n_control_steps):
+            self.control_step()

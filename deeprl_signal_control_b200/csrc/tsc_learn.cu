@@ -1206,17 +1206,24 @@ extern "C" int tscl_host_transition(tscl_handle* h, const float* obs_host, float
   return 0;
 }
 
-// the same hand-over for the device-resident loop (rewards already on the device): one launch instead of six
+// the same hand-over for the device-resident loop (rewards already on the device): one launch instead of six; also the
+// reward store of the IQL replay ring (tscl_iql_transition, tsc_iql.cu)
+int tscl_launch_reward_transition(int device, const float* rew, float* rew_hist, int64_t n_rew, float reward_norm,
+                                  float reward_clip, const float* grew, float* rew_acc, int64_t n, cudaStream_t st) {
+  LCK(cudaSetDevice(device));
+  host_transition_kernel<<<(unsigned)((n_rew + 255) / 256), 256, 0, st>>>(
+      rew, rew_hist, n_rew, reward_norm != 0.f ? 1.0f / reward_norm : 0.f, reward_clip, grew, rew_acc, n);
+  LCK(cudaGetLastError());
+  return 0;
+}
+
 extern "C" int tscl_device_transition(tscl_handle* h, const float* rew_dev, float* rew_hist_dev, int64_t rew_floats,
                                       float reward_norm, float reward_clip, const float* grew_dev, float* rew_acc_dev,
                                       int64_t n, void* stream) {
   if (!h || !rew_dev || !rew_hist_dev || !grew_dev || !rew_acc_dev || rew_floats <= 0 || n <= 0 || n > rew_floats)
     return tsc_set_error("tscl_device_transition: bad argument");
-  LCK(cudaSetDevice(h->device));
-  host_transition_kernel<<<(unsigned)((rew_floats + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-      rew_dev, rew_hist_dev, rew_floats, reward_norm != 0.f ? 1.0f / reward_norm : 0.f, reward_clip, grew_dev, rew_acc_dev, n);
-  LCK(cudaGetLastError());
-  return 0;
+  return tscl_launch_reward_transition(h->device, rew_dev, rew_hist_dev, rew_floats, reward_norm, reward_clip, grew_dev,
+                                       rew_acc_dev, n, (cudaStream_t)stream);
 }
 
 // plain asynchronous copy on a caller-supplied stream (kind: 1 host->device, 2 device->host, 3 device->device)

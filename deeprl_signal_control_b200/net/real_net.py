@@ -424,7 +424,8 @@ def real_net_tables(agent: str = 'ma2c', net_file: str | None = None, flow_rate:
     else from the derived table cache shipped with the package (generated by the same code)."""
     if net_file is not None and os.path.exists(net_file):
         return build_real_net(net_file, flow_rate=flow_rate, agent=agent, coop_gamma=coop_gamma)
-    path = _CACHE % agent
+    # iqll / iqld observe and are rewarded like ia2c (AGENT_MODES, build_obs_program): they share its cache
+    path = _CACHE % ('ia2c' if agent in ('iqll', 'iqld') else agent)
     if not os.path.exists(path):
         raise FileNotFoundError('no Monaco net file given and no derived table cache at %s' % path)
     return load_tables(path)

@@ -226,6 +226,63 @@ int tscl_policy_step_v2r(tscl_handle* h, const float* params, const void* wpack_
  * back-propagate through the rollout's own forward pass instead of recomputing it.
  * bf16 elements per unit in the packed weight image: ((dx+h)/8)*4h*8 + 8*dx*8 */
 
+/* ---- batched independent Q-learning (IQL-LR / IQL-DQN), csrc/tsc_iql.cu ----------------------------------------
+ * Replaces, for R lock-stepped replicas and all A agents at once, the reference's LRQPolicy / DeepQPolicy graphs
+ * (agents/policies.py:285-389), epsilon-greedy acting (agents/models.py:347-362) and ReplayBuffer sampling
+ * (agents/utils.py:231-263).  One Q network per agent, shared by all replicas.
+ *   model 0 (lr):  q = S.Wq + bq
+ *   model 1 (dqn): q = relu(relu([S_wave.Wf + bf | S_wait.Wt + bt]).W0 + b0).Wq + bq   (wait half only when n_w > 0,
+ *                  width num_fc / 4; the wait inputs are the last n_w of the agent's n_s inputs)
+ * Parameters of agent a lie contiguously in [par_off[a], par_off[a+1]) of one flat fp32 vector, in the order and
+ * row-major [in][out] shapes of models.IQL: q_fcw/w, q_fcw/b, (q_fct/w, q_fct/b when n_w > 0), q_fc_0/w, q_fc_0/b,
+ * q/w, q/b (dqn) or q/w, q/b (lr).  Gradients and the Adam moments use the same layout.
+ * Replay ring of C transitions per replica (lock-step: every replica holds the same transition numbers n):
+ *   obs [C+1][R][n_obs]  transition n reads s from slot n % (C+1) and s' from slot (n+1) % (C+1)
+ *   act [C][R][A] int32, rew [C][R][A], done [C] float   transition n sits in slot n % C
+ * n_total transitions have been stored; the live ones are the last min(n_total, C).
+ * Limits (checked by tscl_iql_create): n_s <= 64, max_na <= 8, num_fc <= 128 (a multiple of 4), num_h <= 64. */
+typedef struct tscl_iql_dims {
+  int32_t n_agents;        /* A                                           */
+  int32_t n_obs;           /* row stride of the observation matrix        */
+  int32_t max_na;          /* row stride of the q output                  */
+  int32_t model;           /* 0 = lr, 1 = dqn                             */
+  int32_t num_fc, num_h;   /* dqn widths (ignored for lr)                 */
+  const int32_t* obs_off;  /* [A] first input of agent a in an obs row    */
+  const int32_t* n_s;      /* [A] inputs, wait inputs included            */
+  const int32_t* n_w;      /* [A] wait inputs (dqn only)                  */
+  const int32_t* n_a;      /* [A]                                         */
+  const int64_t* par_off;  /* [A + 1]                                     */
+} tscl_iql_dims;
+
+typedef struct tscl_iql_handle tscl_iql_handle;
+
+int tscl_iql_create(const tscl_iql_dims* dims, int32_t device, tscl_iql_handle** out);
+int tscl_iql_destroy(tscl_iql_handle* h);
+/* obs [R][n_obs] -> act [R][A]: argmax_j q (ties to the lowest j) or, when a uniform draw is < eps, a uniform action in
+ * [0, n_a); draws keyed (seed, step, replica0 + r, agent).  q [R][A][max_na] (zero padded) may be NULL. */
+int tscl_iql_forward(tscl_iql_handle* h, const float* params, const float* obs, int64_t R, float eps, uint64_t seed,
+                     int64_t step, int64_t replica0, int32_t* act, float* q, void* stream);
+/* idx [A][R][B]: B distinct ring slots in [0, size) per (agent, replica), keyed (seed, update, iter, agent,
+ * replica0 + r).  Needs B <= size. */
+int tscl_iql_sample(tscl_iql_handle* h, int64_t R, int32_t B, int64_t size, uint64_t seed, int64_t update, int32_t iter,
+                    int64_t replica0, int32_t* idx, void* stream);
+/* TD loss of the rows selected by idx [A][R][B] (ring slots):  loss_a = scale * sum (q(s)[a] - tq)^2 with
+ * tq = done ? r : r + gamma max q(s') (same weights: no target network).  grads (whole flat vector) = d loss / d params;
+ * stats [A][2] (may be NULL) = {loss_a, scale * sum q(s)[a]}.  Per-CTA partials summed in a fixed order: the same
+ * inputs give the same bits. */
+int tscl_iql_td_grad(tscl_iql_handle* h, const float* params, const float* obs_ring, const int32_t* act_ring,
+                     const float* rew_ring, const float* done_ring, int64_t C, int64_t n_total, int64_t R, int32_t B,
+                     const int32_t* idx, float gamma, float scale, float* grads, float* stats, void* stream);
+/* per-agent clip_by_global_norm(max_norm) (0 = off) + TF1 Adam (beta1 0.9, beta2 0.999, epsilon 1e-8 outside the
+ * sqrt) with lr_t = lr sqrt(1 - beta2^t) / (1 - beta1^t) computed by the caller.  norms [A] (may be NULL) receives the
+ * pre-clip norms. */
+int tscl_iql_clip_adam(tscl_iql_handle* h, float* params, const float* grads, float* m, float* v, float max_norm,
+                       float lr_t, float* norms, void* stream);
+/* reward hand-over into a ring slot, the arithmetic of tscl_device_transition: rew_slot = clip(rew / reward_norm),
+ * rew_acc[0, n) += grew (0 = off for norm / clip) */
+int tscl_iql_transition(tscl_iql_handle* h, const float* rew, float* rew_slot, int64_t rew_floats, float reward_norm,
+                        float reward_clip, const float* grew, float* rew_acc, int64_t n, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
